@@ -5,6 +5,7 @@
   python bench.py --impl reference --gpus N --steps K ...    # the reference's CPU path (C++ restatement) on the host cores
   python bench.py --config 4|5 [--scaling strong]            # the other BASELINE.json sweep configs (default: 2 = configs[1])
   python bench.py --config 3                                 # admission replay: 64-request micro-batches x 200 constraints
+  python bench.py ... --dump-outputs DIR                     # also write the last timed step's results to DIR/*.npy
 
 Workload (config.workload), default: BASELINE.json configs[1] -- "audit sweep: 10 templates, 50 constraints, 1M synthetic
 Pods on 1 B200".  Weak scaling: every rank evaluates its own 1M-Pod shard of the cluster and the violation bitmaps are
@@ -177,9 +178,11 @@ def run_reference(args):
         ref.review_blob(blobs[k % len(blobs)], k8s.AUDIT_EP, cores)
     total_t, total_n = 0.0, 0
     for k in range(steps):
-        _, _, _, secs = ref.review_blob(blobs[(warm + k) % len(blobs)], k8s.AUDIT_EP, cores)
+        pairs, _, _, secs = ref.review_blob(blobs[(warm + k) % len(blobs)], k8s.AUDIT_EP, cores)
         total_t += secs
         total_n += per
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, [[pairs.get(key, 0) for key in ref.constraints()]])
     value = total_n * C / total_t
     tm, cons, nss, mode, n_default, label = workload(cfg)
     sample = (f"oracle/cpu_ref.cpp (C++ restatement of the reference's Client.Review loop: JSON parse, spec.match pre-filter, one Rego evaluation per matching "
@@ -193,6 +196,41 @@ def run_reference(args):
     print(json.dumps(line))
     ref.close()
     return 0
+
+
+# ------------------------------------------------------------------------------------------------ output dump (--dump-outputs)
+DUMP_BYTES = 64 * 1000 * 1000
+
+
+def dump_outputs(out_dir, totals, viol=None, err=None):
+    """What the last timed step handed its caller, as .npy files that two builds can be compared with:
+      totals.npy      float64 [k, C]     per-constraint totals (audit sweep / admission: [violations, matcher errors];
+                                         reference arm: [violating objects])
+      violations.npy  float32 [rows, C]  1 where object row violates constraint c (the uint32 bitmap `viol`, bit c of word c // 32,
+                                         unpacked; with N > 1 the rows of every rank, as gathered)
+      errors.npy      float32 [rows', C] 1 where the matcher errored (`err`: the caller's own rows, the first of viol's)
+      rows.npy        float64 [rows]     the object index of each row
+    Unpacked bits make any difference a whole 1.0.  When every row does not fit in 64 MB, the rows are a fixed seeded sample."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    totals = np.asarray(totals, dtype=np.float64)
+    np.save(os.path.join(out_dir, "totals.npy"), totals)
+    if viol is None:
+        return
+    C = totals.shape[1]
+    per_row = 2 * 4 * C + 8
+    keep = (DUMP_BYTES - totals.nbytes - 4096) // per_row
+    n_rows = len(viol)
+    rows = np.arange(n_rows) if n_rows <= keep else np.sort(np.random.default_rng(0).choice(n_rows, keep, replace=False))
+    cols = np.arange(C)
+
+    def bits(words, idx):
+        w = np.asarray(words).view(np.uint32)[idx]
+        return ((w[:, cols // 32] >> (cols % 32).astype(np.uint32)) & 1).astype(np.float32)
+
+    np.save(os.path.join(out_dir, "violations.npy"), bits(viol, rows))
+    np.save(os.path.join(out_dir, "errors.npy"), bits(err, rows[rows < len(err)]))
+    np.save(os.path.join(out_dir, "rows.npy"), rows.astype(np.float64))
 
 
 # ------------------------------------------------------------------------------------------------ GPU arm: audit sweeps
@@ -275,6 +313,9 @@ def run_ours(args):
     torch.cuda.synchronize()
     if world > 1:
         dist.barrier()
+    if args.dump_outputs and rank == 0:
+        viol = sweep.viol if sweep.gathered is None else sweep.gathered.reshape(-1, words)
+        dump_outputs(args.dump_outputs, sweep.tot[:, :C].cpu().numpy(), viol.cpu().numpy(), sweep.err.cpu().numpy())
     total_ms = ev_a.elapsed_time(ev_b)
     kern_ms = sum(a.elapsed_time(b) for a, b in zip(e0, e1)) / K
     t = torch.tensor([total_ms, kern_ms], dtype=torch.float64, device=dev)
@@ -479,7 +520,7 @@ def run_admission(args):
     sampler = ClockSampler(0)
     sampler.start()
     lat, kern = [], []
-    K = max(args.steps, 50)
+    K = args.steps
     t_all = time.perf_counter()
     for k in range(K):
         arr, nb, _keep = marshalled[k % len(marshalled)]
@@ -489,6 +530,8 @@ def run_admission(args):
         kern.append(resp.stats["kernel_ms"])
     total_s = time.perf_counter() - t_all
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, [resp.totals, resp.err_totals], resp.viol_bits, resp.err_bits)
     def pct(v, p):   # linear interpolation at rank p/100 * (n-1), as gatekeeper_b200/metrics.py (pkg/gator/bench/metrics.go:37-59)
         v = sorted(v)
         r = (p / 100.0) * (len(v) - 1)
@@ -511,7 +554,7 @@ def run_admission(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default: 50 for --config 3, 20 otherwise)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", type=int, default=2, choices=[2, 3, 4, 5], help="BASELINE.json workload: 2 = configs[1] (default), 3 = admission replay, 4 = PSP x mixed GVK, 5 = wildcards")
@@ -523,7 +566,13 @@ def main():
     ap.add_argument("--msg-sample", type=int, default=50_000, help="objects of the sample whose messages are all rendered (e2e.with_messages)")
     ap.add_argument("--spot-check", type=int, default=300, help="objects of the shard checked against the Python oracle inside the run")
     ap.add_argument("--ref-objects-per-step", type=int, default=40_000)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step computed to DIR/*.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 50 if args.config == 3 and args.impl == "ours" else 20
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         sys.exit(run_reference(args))
     if args.config == 3:

@@ -449,23 +449,23 @@ class HostEmuBackend : public Backend {
     const size_t hv = std::hash<std::string>{}(src);
     auto it = cache.find(hv);
     if (it != cache.end()) return it->second;
-    char base[128];
-    snprintf(base, sizeof base, "/tmp/gk_spec_host_%016zx", hv);
-    const std::string so = std::string(base) + ".so";
-    if (access(so.c_str(), R_OK) != 0) {
-      const std::string cpp = std::string(base) + "." + std::to_string((long)getpid()) + ".cpp", tmp = so + "." + std::to_string((long)getpid());
-      {
-        std::ofstream f(cpp);
-        f << src;
-      }
-      const std::string cmd = "g++ -std=c++17 -O1 -w -shared -fPIC -DGK_SPEC_HOST -x c++ " + cpp + " -o " + tmp + " 2> " + cpp + ".log";
-      if (system(cmd.c_str()) != 0) throw BackendError{"GK_SPEC_CHECK: the generated source does not compile for the host: see " + cpp + ".log"};
-      rename(tmp.c_str(), so.c_str());
-      unlink(cpp.c_str());
-      unlink((cpp + ".log").c_str());
+    // compiled in a directory of its own (mkdtemp: a new name, mode 0700), so that only a library this process built is loaded; the
+    // files are removed once loaded (the mapping outlives them), and kept only when the compile fails, for its log
+    const char* td = getenv("TMPDIR");
+    std::string dir = std::string(td && *td ? td : "/tmp") + "/gk_spec_host_XXXXXX";
+    if (!mkdtemp(&dir[0])) throw BackendError{"GK_SPEC_CHECK: cannot create a directory under " + dir.substr(0, dir.rfind('/'))};
+    const std::string cpp = dir + "/spec.cpp", so = dir + "/spec.so", log = dir + "/spec.log";
+    {
+      std::ofstream f(cpp);
+      f << src;
     }
+    const std::string cmd = "g++ -std=c++17 -O1 -w -shared -fPIC -DGK_SPEC_HOST -x c++ '" + cpp + "' -o '" + so + "' 2> '" + log + "'";
+    if (system(cmd.c_str()) != 0) throw BackendError{"GK_SPEC_CHECK: the generated source does not compile for the host: see " + log};
     void* hnd = dlopen(so.c_str(), RTLD_NOW | RTLD_LOCAL);
-    if (!hnd) throw BackendError{std::string("GK_SPEC_CHECK: dlopen: ") + dlerror()};
+    const std::string dl_err = hnd ? "" : dlerror();
+    for (const std::string& f : {so, cpp, log}) unlink(f.c_str());
+    rmdir(dir.c_str());
+    if (!hnd) throw BackendError{"GK_SPEC_CHECK: dlopen: " + dl_err};
     auto fn = reinterpret_cast<SpecHostFn>(dlsym(hnd, "gk_spec_host"));
     if (!fn) throw BackendError{"GK_SPEC_CHECK: gk_spec_host missing"};
     cache[hv] = fn;
